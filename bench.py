@@ -2,7 +2,7 @@
 """bench.py — LM iterations/sec (linearize + damped multifrontal solve + retract + error)
 on the BAL-style workloads of BASELINE.json, through the C-ABI library.
 
-    python bench.py --gpus N --steps K --warmup W [--workload NAME] [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--workload NAME] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one LevenbergMarquardtOptimizer::iterate() from the same initial
 estimate (values restored, lambda reset), i.e. one linearize + >=1 damped
@@ -20,6 +20,11 @@ also solves the same graph unsharded once and the line carries `parity` (sharded
 
 `--impl reference` times the UNMODIFIED reference (oracle/_ref, built from /root/reference by oracle/Makefile;
 falls back to the plain-C oracle port when that binary is absent) on the host cores, on the same workload.
+
+`--dump-outputs DIR` writes, per workload, what the last timed step handed its caller: the packed Values after the
+iterate() (`<workload>_values.npy`, float64; above DUMP_VALUES_MAX entries a fixed, seeded sample of them) and the LM
+error and lambda (`<workload>_error.npy`, `<workload>_lambda.npy`).  The workloads are generated from fixed seeds, so
+two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -41,11 +46,24 @@ REF_EST = {"bal_c3": 2.0, "bal_1m": 9.0, "bal_c4": 40.0, "bal_c5": 200.0, "spher
            "bal_1m_metis": 9.0, "bal_c4_metis": 35.0, "bal_c5_metis": 140.0}
 
 
+def int_at_least(lo):
+    def parse_int(s):
+        v = int(s)
+        if v < lo:
+            raise argparse.ArgumentTypeError(f"must be >= {lo}, got {v}")
+        return v
+    return parse_int
+
+
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
-    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--steps", type=int_at_least(1),
+                    help="timed steps, one LM iterate() each (default 20; --impl reference: as many as fit about 150 s "
+                         "of the reference's iterate())")
+    ap.add_argument("--warmup", type=int_at_least(0),
+                    help="untimed steps before them (default 3, and at least 3 on the GPU; --impl reference: 0 to 3 by "
+                         "the reference's iterate() time)")
     ap.add_argument("--workload", default="auto", help=f"auto = {PRIMARY} (+ {', '.join(SECONDARY)} as other_workloads at N = 1)")
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
@@ -58,7 +76,15 @@ def parse():
                     help="storage of the whitened Jacobians; auto = fp32 for the 10M-factor config (BASELINE configs[4]: "
                          "'FP32 linearize + FP64 solve'), fp64 otherwise")
     ap.add_argument("--jacobian-fp32", action="store_true", help="same as --jacobian fp32")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes what the library computed; --impl reference runs no library step")
+    else:
+        args.steps = 20 if args.steps is None else args.steps
+        args.warmup = 3 if args.warmup is None else args.warmup
+    return args
 
 
 METRIC = "LM iterations/sec (linearize+solve) on BAL-style graph"
@@ -88,6 +114,22 @@ def workload_config(prob, workload, jac32, world, scaling, flush=True):
         f"all-reduce (FP64 sum over NVLink / NVSwitch) of that level's fronts, the owners factor them; back-substitution exchanges the "
         f"owners' solutions per level; one all-reduce of the LM scalars per try; value = iterations/s of the graph actually solved",
     }
+
+
+# float64 entries of one workload's Values written by --dump-outputs (16 MiB): the three workloads of a default run
+# stay under 64 MiB in all
+DUMP_VALUES_MAX = 1 << 21
+
+
+def dump_outputs(outdir, workload, values, error, lam):
+    import numpy as np
+    os.makedirs(outdir, exist_ok=True)
+    if values.size > DUMP_VALUES_MAX:        # same indices at every run: the seed and the size fix them
+        idx = np.sort(np.random.default_rng(0).choice(values.size, DUMP_VALUES_MAX, replace=False))
+        values = values[idx]
+    np.save(os.path.join(outdir, f"{workload}_values.npy"), np.ascontiguousarray(values, dtype=np.float64))
+    np.save(os.path.join(outdir, f"{workload}_error.npy"), np.array([error], dtype=np.float64))
+    np.save(os.path.join(outdir, f"{workload}_lambda.npy"), np.array([lam], dtype=np.float64))
 
 
 # ------------------------------------------------------------------------------------------
@@ -219,8 +261,9 @@ def run_reference(args):
     workload = PRIMARY if args.workload == "auto" else args.workload
     prob, weak = make_problem(args, workload, args.gpus)      # the same graph as the GPU arm at this N
     est = REF_EST.get(workload, 1.0) * (args.gpus if weak else 1)
-    steps = max(1, min(args.steps, int(150.0 / est)))
-    warmup = min(args.warmup, 0 if est > 30 else (1 if est > 1 else 3))
+    # unless given, steps and warm-up are bounded by the reference's iterate() time (bal_c5_metis: 140 s per step)
+    steps = args.steps if args.steps is not None else max(1, min(20, int(150.0 / est)))
+    warmup = args.warmup if args.warmup is not None else (0 if est > 30 else (1 if est > 1 else 3))
     sec, info = reference_time(prob, steps, warmup)
     val = 1.0 / sec
     line = {"metric": METRIC, "value": val, "unit": UNIT, "n_gpus": args.gpus, "steps": steps, "warmup": warmup,
@@ -383,6 +426,11 @@ def measure(args, workload, ctx, dist, rank, local, world, primary):
     steps = args.steps
     ms, wall, launches = timed(step_resident, steps, max(3, args.warmup), prepare=prepare_resident)
     clocks = sampler.stop(tuple(timed.region)) if (rank == 0 and primary) else None
+    if args.dump_outputs:
+        out_values = dev.get_values_all() if world > 1 else dev.get_values()    # (get_values_all is collective)
+        if rank == 0:
+            out_state = lm._state()
+            dump_outputs(args.dump_outputs, workload, out_values, out_state.error, out_state.lambda_)
     ms_e2e, wall_e2e, _ = timed(step_e2e, steps, 1)
     ms_warm, _, _ = timed(step_resident, steps, 1, flush=False, prepare=prepare_resident)   # information only: L2 left warm between iterations
 
